@@ -8,6 +8,7 @@ shard in HBM and a batch of 512; the two flat gradient blocks are all-reduced ov
   python bench.py --impl reference ...                   # the reference's CPU implementation (oracle port)
   python bench.py --config cfg2|cfg1                     # BASELINE.json configs[1] / configs[0] shapes
   python bench.py --config replay                        # configs[3]: 250k stored sequence starts per GPU, sample / update
+  python bench.py --dump-outputs DIR                     # also write the last timed step's outputs (Arm.dump_outputs)
 
 A step = one pass of learner.py:84-139: prioritized sample from the HBM replay shard -> gather -> target/online
 chains -> TD/priority kernels -> critic BPTT + Adam -> actor chain -> DPG backward + Adam -> priority write-back into
@@ -269,12 +270,22 @@ class Arm:
         self.episodes = episodes
         self.rp = build_replay(engine_mod, self.cfg, episodes, self.ep_len, seed=seed_base + rank, device=dev)
         self.gen = torch.Generator(device=dev).manual_seed(1234 + rank)
+        # what the resident loop writes back into the tree: see _next_batch
+        self.written_prio = 0.01 + 0.99 * torch.rand(self.cfg.batch, device=dev,
+                                                     generator=torch.Generator(device=dev).manual_seed(4321 + rank))
 
     def _next_batch(self, eng, used):
         """LearnerEngine.step's prefetch hook: tree write-back of the batch just used (learner.py:136-139), then the
         sum-tree draw + gather of the next one (learner.py:84) - the same work per iteration as the sequential loop,
-        issued as soon as the priorities exist so that the next batch's target chains can run mid-iteration."""
-        self.rp.update_priorities(used.leaf_idx, used.priority)
+        issued as soon as the priorities exist so that the next batch's target chains can run mid-iteration.
+
+        The write-back scatters a fixed, seeded priority vector into the trained leaves rather than the priorities the
+        step computed: the same kernel, element count and bytes, so the same cost.  Computed priorities carry the
+        rounding of the build (split-K and reduction atomics), and written back they would steer every later draw:
+        two runs, or two builds, would train on different batches after a few dozen steps.  This way the batches
+        depend on the seeds alone and the outputs of any step can be compared (dump_outputs)."""
+        self.rp.update_priorities(used.leaf_idx, self.written_prio)
+        self.trained_leaf_idx = used.leaf_idx    # slot of the batch just trained on: the next draw fills the other one
         self.rp.sample_into(eng, generator=self.gen)
 
     def step_resident(self):
@@ -370,6 +381,23 @@ class Arm:
         copy_stream.synchronize()
         return ev0.elapsed_time(ev1) / steps, h2d, d2h
 
+    def dump_outputs(self, out_dir):
+        """What the last resident step handed its caller, as DIR/<name>.npy: q / target / squared TD / priorities /
+        losses of the iteration, the actor and critic weights after its updates, and the replay rows it trained on
+        (float64 indices).  About 25 MB at cfg3, the largest configuration.
+
+        Replay shard, weights, uniforms and the priorities written back are seeded (_next_batch), so runs with the
+        same arguments train on the same batches; their outputs differ by the rounding of the atomics only."""
+        self.eng.flush()
+        torch.cuda.synchronize()
+        eng = self.eng
+        arrays = {"q_value": eng.q_value, "target_q_value": eng.target_q_value, "td_sq": eng.td_sq,
+                  "priority": eng.priority, "losses": eng.losses, "actor_params": eng.flat["actor"],
+                  "critic_params": eng.flat["critic"], "leaf_idx": self.trained_leaf_idx.double()}
+        os.makedirs(out_dir, exist_ok=True)
+        for name, t in arrays.items():
+            np.save(os.path.join(out_dir, name + ".npy"), t.detach().cpu().numpy())
+
     @property
     def launches_per_step(self):
         return self.eng.launches_per_iteration + 2 + 1   # + tree_sample, gather_batch + tree_update
@@ -440,6 +468,21 @@ def scan_roofline(nv, c, dev, peaks, ms_iter):
                                 "frac_of_sustained_peak": flops_it / (ms_iter * 1e-3) / 1e12 / peaks["bf16_sustained"]}}
 
 
+def dump_replay_outputs(out_dir, rp, eng, n_cols=64):
+    """What the replay legs hand their caller, as DIR/<name>.npy: the last timed draw (leaf indices, float64, and
+    the gathered batch of a fixed, seeded sample of n_cols of its sequences - the whole batch is ~100 MB at cfg3) and
+    the tree after the timed priority updates (its total, float64, and its level above the leaves)."""
+    torch.cuda.synchronize()
+    cols = np.sort(np.random.default_rng(0).choice(eng.cfg.batch, n_cols, replace=False))
+    idx = torch.as_tensor(cols, device=eng.leaf_idx.device)
+    arrays = {"leaf_idx": eng.leaf_idx.double(), "obs": eng.obs[:, idx], "act": eng.act[:, idx], "rew": eng.rew[:, idx],
+              "term": eng.term[:, idx], "states": eng.states[:, :, idx], "tree_level1": rp.tree_level(1),
+              "total_priority": torch.tensor([rp.stats()["total_priority"]], dtype=torch.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().cpu().numpy())
+
+
 def run_replay_bench(args, engine, dev, world, rank, dist, barrier):
     """BASELINE.json configs[3]: GPU-resident prioritized replay, 2 M stored sequence starts sharded 8-way = 250 k starts
     per GPU (1000 episodes x 250 starts, Humanoid row widths): sum-tree sample + gather and priority-update throughput,
@@ -471,7 +514,7 @@ def run_replay_bench(args, engine, dev, world, rank, dist, barrier):
     gen = torch.Generator(device=dev).manual_seed(rank)
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     B = cfg.batch
-    steps, warm = max(args.steps, 50), max(args.warmup, 5)
+    steps, warm = args.steps, max(args.warmup, 5)
     for _ in range(warm):
         rp.sample_into(eng, generator=gen)
     barrier()
@@ -493,7 +536,7 @@ def run_replay_bench(args, engine, dev, world, rank, dist, barrier):
     exact = exact_after = None
     if rank == 0:   # same uniforms, same tree: identical flat indices from the CUDA tree and its C restatement
         exact = bool(np.array_equal(leaf.cpu().numpy(), oracle.sample(u.cpu().numpy())))
-    prio = torch.rand(B, device=dev)
+    prio = torch.rand(B, device=dev, generator=gen)
     for _ in range(warm):
         rp.update_priorities(eng.leaf_idx, prio)
     barrier()
@@ -507,6 +550,8 @@ def run_replay_bench(args, engine, dev, world, rank, dist, barrier):
         oracle.update_batch(eng.leaf_idx.cpu().numpy(), prio.cpu().numpy())
         u2 = torch.rand(100000, device=dev, generator=gen)
         exact_after = bool(np.array_equal(rp.sample_indices(u2).cpu().numpy(), oracle.sample(u2.cpu().numpy())))
+    if args.dump_outputs and rank == 0:
+        dump_replay_outputs(args.dump_outputs, rp, eng)
     t = torch.tensor([ms_sample, ms_update], device=dev)
     if dist is not None:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -536,7 +581,8 @@ def main():
     _claim_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=100,
+                    help="timed steps of every leg (headline, host-fed, strong-scaling, secondary configs, replay)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default="cfg3", choices=sorted(CONFIGS) + ["replay"])
@@ -544,7 +590,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary configs / strong-scaling legs (profiling runs)")
     ap.add_argument("--cpu-steps", type=int, default=4)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (rank 0), to compare two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        # the CPU port stops on a wall-clock budget: how many iterations it ran, and so its last outputs, vary
+        ap.error("--dump-outputs writes the outputs of the B200 arm: not with --impl reference")
     if args.warmup < 3:
         args.warmup = 3
     name = args.config if args.config != "replay" else "cfg3"
@@ -588,6 +641,8 @@ def main():
     log("HBM-resident arm")
     ms = arm.time_resident(args.steps, args.warmup, barrier, clocks)
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        arm.dump_outputs(args.dump_outputs)
 
     def max_over_ranks(x):
         t = torch.tensor([x], device=dev)
@@ -619,7 +674,7 @@ def main():
         log("strong-scaling leg")
         cs = dict(c, batch=B // world)
         arm_s = Arm(engine, cs, dev, rank, max(64, args.episodes // world), data_parallel=True, seed_base=500)
-        ms_s = max_over_ranks(arm_s.time_resident(max(20, args.steps // 2), args.warmup, barrier))
+        ms_s = max_over_ranks(arm_s.time_resident(args.steps, args.warmup, barrier))
         strong = {"global_batch": B, "per_gpu_batch": B // world, "ms_per_step": ms_s,
                   "value": B * L / (ms_s * 1e-3), "unit": "seq-steps/s",
                   "replicas_identical": arm_s.eng.replicas_identical()}
@@ -632,7 +687,7 @@ def main():
                 continue
             log(f"secondary config {oname}")
             arm_o = Arm(engine, CONFIGS[oname], dev, rank, 128, data_parallel=True, seed_base=900)
-            ms_o = max_over_ranks(arm_o.time_resident(50, 5, barrier))
+            ms_o = max_over_ranks(arm_o.time_resident(args.steps, args.warmup, barrier))
             co = CONFIGS[oname]
             others[oname] = {"workload": workload_string(oname, co), "ms_per_step": ms_o,
                              "value": world * co["batch"] * co["learning"] / (ms_o * 1e-3), "unit": "seq-steps/s",

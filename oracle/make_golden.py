@@ -18,11 +18,16 @@ Files
   ref_ingest.npz        the real LearnerReplayMemory.load (replay_memory.py:138-157) over a deterministic sequence of actor
                         files with a small sequence cap: sequence_counter and surviving episodes after every file
   ref_actor_prio.npz    the real Actor.calc_nstep_reward / Actor.calc_priorities (actor.py:74-107) on synthetic
-                        episodes of several lengths: raw and n-step rewards, weights of the three nets the
-                        pass reads, and the initial priorities it produced (next-row N2 of SURVEY 8f)
+                        episodes of several lengths: raw and n-step rewards, torch seed and weight digests of
+                        the three nets the pass reads, and the initial priorities it produced (next-row N2 of
+                        SURVEY 8f)
+Inputs that the tests can rebuild - initial weights from the torch seed with the oracle/ref_port.py nets, sampled
+batches from the synthetic actor file and the drawn (episode, sequence) indices - are stored as SHA-256 digests
+(array_digest), and the rebuilt arrays are checked against them bit for bit.
 """
 from __future__ import annotations
 
+import hashlib
 import os
 import sys
 
@@ -37,39 +42,62 @@ from oracle import ref_harness, ref_port  # noqa: E402
 
 OUT = os.path.join(ROOT, "tests", "golden")
 NETS = ("actor", "critic")
+BATCH_KEYS = ("obs", "act", "rew", "term", "a_state", "ta_state", "c_state", "tc_state")
+SAMPLE = 4096          # elements kept of a full gradient / weight tensor of the iterations in `full_iters`
+
+
+def array_digest(a) -> str:
+    """SHA-256 of dtype, shape and bytes: lets a fixture pin an input that the tests rebuild (initial weights from
+    the torch seed, sampled batches from the synthetic actor file) bit for bit without storing it."""
+    a = np.ascontiguousarray(a)
+    return hashlib.sha256(f"{a.dtype.str}{a.shape}".encode() + a.tobytes()).hexdigest()
+
+
+def _sample_index(n):
+    """Sorted, seeded sample of SAMPLE flat positions (all of them for a smaller tensor), stored with the values."""
+    if n <= SAMPLE:
+        return np.arange(n, dtype=np.int32)
+    return np.sort(np.random.default_rng(n).choice(n, SAMPLE, replace=False)).astype(np.int32)
 
 
 def _flatten(records, full_iters=(0,)):
+    """Everything the reference computed, with its inputs (initial weights, batches) as digests and the full
+    gradient / weight tensors of `full_iters` as a fixed sample: every fixture stays under 1 MB."""
     out = {"n_iters": np.int64(len(records)), "torch_version": np.array(torch.__version__)}
     r0 = records[0]
     for net in NETS:
         for k, v in r0[f"{net}_init"].items():
-            out[f"init/{net}/{k}"] = v
+            out[f"init_sha256/{net}/{k}"] = np.array(array_digest(v))
     for i, r in enumerate(records):
-        for k in ("obs", "act", "rew", "term", "a_state", "ta_state", "c_state", "tc_state",
-                  "episode_index", "sequence_index", "q_value", "target_q_value", "critic_loss",
+        for k in BATCH_KEYS:
+            out[f"it{i}/sha256/{k}"] = np.array(array_digest(r[k]))
+        for k in ("episode_index", "sequence_index", "q_value", "target_q_value", "critic_loss",
                   "actor_loss", "average_td_loss", "priority_written", "total_priority_written"):
             out[f"it{i}/{k}"] = np.asarray(r[k])
         for net in NETS:
             for k, v in r[f"{net}_grad"].items():
                 if i in full_iters:
-                    out[f"it{i}/{net}_grad/{k}"] = v
+                    idx = _sample_index(v.size)
+                    out[f"it{i}/sample_idx/{net}/{k}"] = idx
+                    out[f"it{i}/{net}_grad/{k}"] = v.reshape(-1)[idx]
                 out[f"it{i}/{net}_grad_norm/{k}"] = np.float64(np.linalg.norm(v.astype(np.float64)))
             for k, v in r[f"{net}_after"].items():
                 if i in full_iters:
-                    out[f"it{i}/{net}_after/{k}"] = v
+                    out[f"it{i}/{net}_after/{k}"] = v.reshape(-1)[out[f"it{i}/sample_idx/{net}/{k}"]]
                 out[f"it{i}/{net}_after_norm/{k}"] = np.float64(np.linalg.norm(v.astype(np.float64)))
                 out[f"it{i}/{net}_after_sub/{k}"] = v.reshape(-1)[::97].copy()
     return out
 
 
 def gen_learner(name, models_module=None, **kw):
-    recs, times, _ = ref_harness.run_reference_learner(models_module=models_module, **kw)
+    recs, times, lr = ref_harness.run_reference_learner(models_module=models_module, **kw)
     d = _flatten(recs)
     d["config"] = np.array(repr(kw))
-    for k in ("obs_size", "n_actions", "hidden", "batch_size", "burn_in", "learning", "n_step"):
+    for k in ("obs_size", "n_actions", "hidden", "batch_size", "burn_in", "learning", "n_step", "seed", "data_seed",
+              "episode_len"):
         d[f"cfg/{k}"] = np.int64(kw.get(k, {"hidden": 128, "batch_size": 32, "burn_in": 20,
-                                          "learning": 40, "n_step": 5}.get(k, 0)))
+                                          "learning": 40, "n_step": 5, "episode_len": 250}.get(k, 0)))
+    d["cfg/n_episodes"] = np.int64(len(lr.memory.memory))      # the one actor file the batches were drawn from
     path = os.path.join(OUT, name)
     np.savez_compressed(path, **d)
     print(name, "iters", len(recs), "iter-times", np.round(times, 3), "size %.2f MB" % (os.path.getsize(path) / 1e6))
@@ -227,9 +255,10 @@ def gen_actor_priorities():
             # weights so that the fixture distinguishes the four roles
             a.target_actor = ref_models.ActorNet(O, A, 0).eval()
             a.target_critic = ref_models.CriticNet(O, A, 0).eval()
+            d[f"c{ci}/seed"] = np.int64(100 + ci)
             for net_name in ("critic", "target_actor", "target_critic"):
                 for k, v in getattr(a, net_name).state_dict().items():
-                    d[f"c{ci}/{net_name}/{k}"] = v.detach().clone().numpy()
+                    d[f"c{ci}/{net_name}/{k}"] = np.array(array_digest(v.detach().numpy()))
             d[f"c{ci}/cfg"] = np.int64([O, A, 128, a.burn_in_length, a.learning_length, a.n_step])
             d[f"c{ci}/gamma"] = np.float64(a.gamma)
             d[f"c{ci}/n_episodes"] = np.int64(len(lens))

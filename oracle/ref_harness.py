@@ -1,9 +1,8 @@
 """Oracle harness: run the UNMODIFIED reference learner loop on CPU (this container only).
 
 TEST INFRASTRUCTURE - never imported by the product path.  Only `oracle/make_golden.py`
-(fixture generation, run in the build container where /root/reference is mounted) uses it.
-/root/reference does not exist on the GPU box, so nothing under tests/ -m gpu, smoke() or
-bench.py may import this module.
+(fixture generation) runs it, on a machine that has the reference sources (R2D2_REFERENCE_DIR).
+Importing it needs no reference; the tests, smoke() and bench.py never call into it.
 
 What it does (SURVEY.md section 8c / Appendix A):
   * puts stub modules for `dm_control`, `dm_control.suite`, `gym`, `PIL` in sys.modules
@@ -26,10 +25,12 @@ import collections
 import os
 import sys
 import types
-from collections import OrderedDict, deque
+from collections import OrderedDict
 
 import numpy as np
 import torch
+
+from oracle import ref_port
 
 REFERENCE_DIR = os.environ.get("R2D2_REFERENCE_DIR", "/root/reference")
 
@@ -74,34 +75,9 @@ def _install_stubs(obs_size: int, n_actions: int):
             sys.modules["PIL.Image"] = pil.Image
 
 
-def make_actor_file(path, *, obs_size, n_actions, hidden, n_episodes, episode_len, seed,
-                    burn_in, learning, n_step):
-    """Synthetic memory{i}.pt in the actor format (actor.py:163-176, replay_memory.py:55-59).
-
-    Episode = `episode_len` real rows + n_step pad rows (zeros, reward [0.], terminal [1.],
-    actor.py:173).  len(priority[ep]) = episode_len - (burn_in+learning) (actor.py:106-107).
-    Rewards are treated as already n-step pre-summed (actor.py:74-76)."""
-    rng = np.random.default_rng(seed)
-    seq_len = burn_in + learning
-    mem, states, prios, totals = deque(), deque(), deque(), []
-    for _ in range(n_episodes):
-        ep = []
-        for _t in range(episode_len):
-            ep.append((rng.standard_normal(obs_size).astype(np.float32),
-                       rng.uniform(-1, 1, n_actions).astype(np.float32),
-                       [float(np.float32(rng.standard_normal()))], [0.0]))
-        for _t in range(n_step):
-            ep.append((np.zeros(obs_size, np.float32), np.zeros(n_actions, np.float32), [0.0], [1.0]))
-        st = [[[(0.1 * rng.standard_normal(hidden)).astype(np.float32),
-                (0.1 * rng.standard_normal(hidden)).astype(np.float32)] for _net in range(4)]
-              for _t in range(episode_len)]
-        pr = [float(np.float32(rng.uniform(0.01, 1.0))) for _ in range(episode_len - seq_len)]
-        mem.append(ep)
-        states.append(st)
-        prios.append(pr)
-        totals.append(sum(pr))
-    torch.save({"replay_memory": mem, "recurrent_state": states, "priority": prios,
-                "total_priority": totals}, path)
+def make_actor_file(path, **kw):
+    """Synthetic memory{i}.pt in the actor format (oracle/ref_port.py synthetic_actor_file)."""
+    torch.save(ref_port.synthetic_actor_file(**kw), path)
 
 
 def run_reference_learner(*, obs_size, n_actions, hidden=128, batch_size=32, burn_in=20,

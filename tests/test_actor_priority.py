@@ -7,14 +7,23 @@
 import numpy as np
 import pytest
 
-from conftest import load_golden, rel_l2
+from conftest import checked_state, load_golden, rel_l2
 
-KEYS = ("l1.weight", "l1.bias", "l2.weight_ih", "l2.weight_hh", "l2.bias_ih", "l2.bias_hh", "l3.weight", "l3.bias")
+def _nets(g, ci, O, A, H):
+    """The three nets the reference's pass read: under its torch seed the actor builds actor, critic, then the fixture
+    target actor, target critic (oracle/make_golden.py gen_actor_priorities); the port's nets draw the same weights."""
+    import torch
+    from oracle import ref_port
+    torch.manual_seed(int(g[f"c{ci}/seed"]))
+    ref_port.PortActorNet(O, A, 0, H)
+    made = {"critic": ref_port.PortCriticNet(O, A, 0, H), "target_actor": ref_port.PortActorNet(O, A, 0, H),
+            "target_critic": ref_port.PortCriticNet(O, A, 0, H)}
+    return {net: checked_state(g, f"c{ci}/{net}", m) for net, m in made.items()}
 
 
 def _case(g, ci):
     O, A, H, Bn, L, n = (int(x) for x in g[f"c{ci}/cfg"])
-    nets = {net: {k: g[f"c{ci}/{net}/{k}"] for k in KEYS} for net in ("critic", "target_actor", "target_critic")}
+    nets = _nets(g, ci, O, A, H)
     eps = []
     for ei in range(int(g[f"c{ci}/n_episodes"])):
         eps.append({k: g[f"c{ci}/e{ei}/{k}"] for k in ("obs", "act", "rew_raw", "rew_nstep", "term", "priority")})

@@ -11,7 +11,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import golden_batch, golden_params, load_golden, rel_l2
+from conftest import golden_batch, golden_init, golden_sample, load_golden, rel_l2
 from oracle import ref_port
 
 pytestmark = pytest.mark.gpu
@@ -40,7 +40,7 @@ def test_against_reference_goldens(eng_mod, name):
     g = load_golden(name)
     cfg = _cfg(eng_mod, g)
     eng = eng_mod.LearnerEngine(cfg)
-    eng.load_state_dicts(golden_params(g, "init/actor"), golden_params(g, "init/critic"))
+    eng.load_state_dicts(*golden_init(g))
     report = []
     for it in range(int(g["n_iters"])):
         eng.set_batch(golden_batch(g, it))
@@ -62,8 +62,8 @@ def test_against_reference_goldens(eng_mod, name):
                 errs[f"{net}_gnorm/{k}"] = abs(np.linalg.norm(gr[k].astype(np.float64)) - gn) / max(gn, 1e-30)
                 errs[f"{net}_after_sub/{k}"] = rel_l2(pa[k].reshape(-1)[::97], g[f"it{it}/{net}_after_sub/{k}"])
                 if it == 0:
-                    errs[f"{net}_grad/{k}"] = rel_l2(gr[k], g[f"it0/{net}_grad/{k}"])
-                    errs[f"{net}_after/{k}"] = rel_l2(pa[k], g[f"it0/{net}_after/{k}"])
+                    errs[f"{net}_grad/{k}"] = rel_l2(golden_sample(g, 0, net, k, gr[k]), g[f"it0/{net}_grad/{k}"])
+                    errs[f"{net}_after/{k}"] = rel_l2(golden_sample(g, 0, net, k, pa[k]), g[f"it0/{net}_after/{k}"])
         report.append(errs)
         bad = {k: v for k, v in errs.items() if not v < TOL}
         assert not bad, f"{name} iteration {it}: {bad}"

@@ -4,35 +4,28 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import golden_batch, golden_params, load_golden, rel_l2
+from conftest import checked_state, golden_batch, golden_cfg, golden_init, golden_sample, load_golden, rel_l2
 from oracle import learner_oracle as lo
 from oracle import ref_port
 
 CASES = [("ref_walker_h128.npz", 1), ("ref_pend_h128.npz", 2), ("ref_tiny_h32.npz", 4)]
 
 
-def _cfg(g):
-    return ref_port.PathConfig(obs=int(g["cfg/obs_size"]), act=int(g["cfg/n_actions"]), hidden=int(g["cfg/hidden"]),
-                               batch=int(g["cfg/batch_size"]), burn_in=int(g["cfg/burn_in"]),
-                               learning=int(g["cfg/learning"]), n_step=int(g["cfg/n_step"]))
-
-
 @pytest.mark.parametrize("name,seed", CASES)
 def test_port_init_bit_identical(name, seed):
     """Same torch seed -> the port's nets equal the reference's models.py nets bit for bit."""
     g = load_golden(name)
-    lr = ref_port.PortLearner(_cfg(g), seed=seed)
+    lr = ref_port.PortLearner(golden_cfg(g), seed=seed)
     for net, mod in (("actor", lr.actor), ("critic", lr.critic)):
-        for k, v in mod.state_dict().items():
-            assert np.array_equal(v.numpy(), g[f"init/{net}/{k}"]), (net, k)
+        checked_state(g, f"init_sha256/{net}", mod)
 
 
 @pytest.mark.parametrize("name,seed", CASES)
 def test_port_iterations_match_reference(name, seed):
     g = load_golden(name)
     torch.set_num_threads(4)
-    lr = ref_port.PortLearner(_cfg(g))
-    lr.load_params(golden_params(g, "init/actor"), golden_params(g, "init/critic"))
+    lr = ref_port.PortLearner(golden_cfg(g))
+    lr.load_params(*golden_init(g))
     for it in range(int(g["n_iters"])):
         out = lr.iteration(golden_batch(g, it))
         assert rel_l2(out["q_value"], g[f"it{it}/q_value"]) < 2e-6
@@ -48,17 +41,17 @@ def test_port_iterations_match_reference(name, seed):
         if it == 0:
             for net in ("actor", "critic"):
                 for k in ref_port.PARAM_KEYS:
-                    assert rel_l2(out[f"{net}_grad"][k], g[f"it0/{net}_grad/{k}"]) < 1e-4, (net, k)
-                    assert rel_l2(out[f"{net}_after"][k], g[f"it0/{net}_after/{k}"]) < 1e-6, (net, k)
+                    assert rel_l2(golden_sample(g, 0, net, k, out[f"{net}_grad"][k]), g[f"it0/{net}_grad/{k}"]) < 1e-4, (net, k)
+                    assert rel_l2(golden_sample(g, 0, net, k, out[f"{net}_after"][k]), g[f"it0/{net}_after/{k}"]) < 1e-6, (net, k)
 
 
 @pytest.mark.parametrize("name,seed", CASES)
 def test_numpy_oracle_matches_reference(name, seed):
     """float64 manual-BPTT oracle vs the reference's fp32 autograd: agreement at fp32 round-off."""
     g = load_golden(name)
-    c = _cfg(g)
-    ol = lo.OracleLearner(golden_params(g, "init/actor"), golden_params(g, "init/critic"), burn_in=c.burn_in,
-                          learning=c.learning, n_step=c.n_step)
+    c = golden_cfg(g)
+    init = dict(zip(("actor", "critic"), golden_init(g)))
+    ol = lo.OracleLearner(init["actor"], init["critic"], burn_in=c.burn_in, learning=c.learning, n_step=c.n_step)
     for it in range(int(g["n_iters"])):
         out = ol.iteration(golden_batch(g, it))
         assert rel_l2(out["q_value"], g[f"it{it}/q_value"]) < 5e-5
@@ -70,10 +63,11 @@ def test_numpy_oracle_matches_reference(name, seed):
         if it == 0:
             for net in ("actor", "critic"):
                 for k in lo.PARAM_KEYS:
-                    assert rel_l2(out[f"{net}_grad"][k], g[f"it0/{net}_grad/{k}"]) < 2e-4, (net, k)
+                    assert rel_l2(golden_sample(g, 0, net, k, out[f"{net}_grad"][k]), g[f"it0/{net}_grad/{k}"]) < 2e-4, (net, k)
                     # Adam's first step is sign-like (|update| = lr); compare the update, not the params
-                    upd = out[f"{net}_after"][k] - g[f"init/{net}/{k}"]
-                    ref_upd = g[f"it0/{net}_after/{k}"].astype(np.float64) - g[f"init/{net}/{k}"]
+                    init0 = golden_sample(g, 0, net, k, init[net][k])
+                    upd = golden_sample(g, 0, net, k, out[f"{net}_after"][k]) - init0
+                    ref_upd = g[f"it0/{net}_after/{k}"].astype(np.float64) - init0
                     assert rel_l2(upd, ref_upd) < 5e-2, (net, k)
         for net in ("actor", "critic"):
             for k in lo.PARAM_KEYS:
