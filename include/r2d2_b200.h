@@ -99,7 +99,9 @@ int r2d2_debug_scan_forward_trace(const float* gin, const float* whh, float* gat
 int r2d2_debug_scan_backward_trace(const float* gates, const float* hs, const float* cs, const float* whh,
                                    const float* dh_head, float* dgates, int T, int B, int H, long long* trace,
                                    r2d2_stream_t stream);
-/* debug: clusters of the tcgen05 scan kernel the device can keep resident at once (-1 if not instantiated) */
+/* debug: clusters of a tcgen05 scan kernel the device can keep resident at once (-1 if not instantiated):
+ * H in {32,64,128,256,512}, nb = 16 or 32 rows per tile (the kernels the batch tiling chooses between, forward or
+ * backward); H = 512, nb = 80, backward = 0 is the H = 512 forward kernel of up to 80 rows per cluster. */
 int r2d2_debug_max_active_clusters(int H, int nb, int backward);
 /* GEMM implementation switch for A/B checks: 1 = tcgen05/TMEM with skinny problems (K<64, N<32 or M<32) on the
  * single-launch mma.sync kernel (default), 2 = tcgen05 for every shape, 0 = mma.sync v1 kernel only */

@@ -34,20 +34,18 @@ def value_rescale(x):
     return np.sign(x) * (np.sqrt(np.abs(x) + 1.0) - 1.0)
 
 
-def net_forward(p, x, h0, c0, *, critic: bool, repeat: int = 1):
-    """x [T,B,I] -> saved activations.  steps = T*repeat; step s consumes row s//repeat.
-    Saved: z1 [T,B,H]; gates [S,B,4H] post-activation (i,f,g,o); hs, cs [S+1,B,H] (slot 0 = initial
-    state); out [S,B,A]."""
-    T, B, _ = x.shape
-    H = p["l2.weight_hh"].shape[1]
-    z1 = np.tanh(x @ p["l1.weight"].T + p["l1.bias"])
-    gin = z1 @ p["l2.weight_ih"].T + (p["l2.bias_ih"] + p["l2.bias_hh"])
+def scan_forward(gin, whh, h0, c0, repeat: int = 1):
+    """The serial LSTM scan alone.  gin [T,B,4H] = input projection + both biases, whh [4H,H], h0/c0 [B,H].
+    steps S = T*repeat; step s consumes row s//repeat.  Returns gates [S,B,4H] post-activation (i,f,g,o) and
+    hs, cs [S+1,B,H] (slot 0 = initial state)."""
+    T, B, G = gin.shape
+    H = G // 4
     S = T * repeat
-    hs = np.zeros((S + 1, B, H), x.dtype)
-    cs = np.zeros((S + 1, B, H), x.dtype)
-    gates = np.zeros((S, B, 4 * H), x.dtype)
+    hs = np.zeros((S + 1, B, H), gin.dtype)
+    cs = np.zeros((S + 1, B, H), gin.dtype)
+    gates = np.zeros((S, B, 4 * H), gin.dtype)
     hs[0], cs[0] = h0, c0
-    whh_t = p["l2.weight_hh"].T
+    whh_t = whh.T
     for s in range(S):
         g = gin[s // repeat] + hs[s] @ whh_t
         i, f, gg, o = (_sigmoid(g[:, :H]), _sigmoid(g[:, H:2 * H]), np.tanh(g[:, 2 * H:3 * H]),
@@ -55,6 +53,39 @@ def net_forward(p, x, h0, c0, *, critic: bool, repeat: int = 1):
         cs[s + 1] = f * cs[s] + i * gg
         hs[s + 1] = o * np.tanh(cs[s + 1])
         gates[s] = np.concatenate((i, f, gg, o), 1)
+    return gates, hs, cs
+
+
+def scan_backward(gates, cs, whh, d_h_head):
+    """BPTT of scan_forward.  d_h_head [S,B,H] = dLoss/dh_s from outside the recurrence (zero rows where
+    there is none).  Returns d_gates [S,B,4H] (w.r.t. the pre-activations), dh0, dc0 [B,H]."""
+    S, B, G = gates.shape
+    H = G // 4
+    d_gates = np.zeros_like(gates)
+    dh_rec = np.zeros((B, H), gates.dtype)
+    dc_next = np.zeros((B, H), gates.dtype)
+    for s in range(S - 1, -1, -1):
+        i, f, gg, o = (gates[s][:, :H], gates[s][:, H:2 * H], gates[s][:, 2 * H:3 * H], gates[s][:, 3 * H:])
+        tc = np.tanh(cs[s + 1])
+        dh = d_h_head[s] + dh_rec
+        d_o = dh * tc * o * (1.0 - o)
+        dc = dc_next + dh * o * (1.0 - tc * tc)
+        d_i = dc * gg * i * (1.0 - i)
+        d_f = dc * cs[s] * f * (1.0 - f)
+        d_g = dc * i * (1.0 - gg * gg)
+        dc_next = dc * f
+        d_gates[s] = np.concatenate((d_i, d_f, d_g, d_o), 1)
+        dh_rec = d_gates[s] @ whh
+    return d_gates, dh_rec, dc_next
+
+
+def net_forward(p, x, h0, c0, *, critic: bool, repeat: int = 1):
+    """x [T,B,I] -> saved activations.  steps = T*repeat; step s consumes row s//repeat.
+    Saved: z1 [T,B,H]; gates [S,B,4H] post-activation (i,f,g,o); hs, cs [S+1,B,H] (slot 0 = initial
+    state); out [S,B,A]."""
+    z1 = np.tanh(x @ p["l1.weight"].T + p["l1.bias"])
+    gin = z1 @ p["l2.weight_ih"].T + (p["l2.bias_ih"] + p["l2.bias_hh"])
+    gates, hs, cs = scan_forward(gin, p["l2.weight_hh"], h0, c0, repeat)
     if critic:
         out = hs[1:] @ p["l3.weight"].T + p["l3.bias"]
     else:
@@ -69,6 +100,8 @@ def net_backward(p, sv, d_out, *, critic: bool, want_wgrad: bool = True, want_dx
     T = S // repeat
     H = hs.shape[2]
     g = {}
+    # weight gradients contract over (step, batch): tensordot runs them as one matrix product each
+    wgrad = lambda a, b: np.tensordot(a, b, axes=([0, 1], [0, 1]))  # noqa: E731
     if critic:
         d_pre = d_out
         head_in = hs[1:]
@@ -78,33 +111,18 @@ def net_backward(p, sv, d_out, *, critic: bool, want_wgrad: bool = True, want_dx
         head_in = np.tanh(hs[1:])
         d_h_head = (d_pre @ p["l3.weight"]) * (1.0 - head_in * head_in)
     if want_wgrad:
-        g["l3.weight"] = np.einsum("sba,sbh->ah", d_pre, head_in)
+        g["l3.weight"] = wgrad(d_pre, head_in)
         g["l3.bias"] = d_pre.sum((0, 1))
-    d_gates = np.zeros_like(gates)
-    dh_rec = np.zeros((B, H), x.dtype)
-    dc_next = np.zeros((B, H), x.dtype)
-    whh = p["l2.weight_hh"]
-    for s in range(S - 1, -1, -1):
-        i, f, gg, o = (gates[s][:, :H], gates[s][:, H:2 * H], gates[s][:, 2 * H:3 * H], gates[s][:, 3 * H:])
-        tc = np.tanh(cs[s + 1])
-        dh = d_h_head[s] + dh_rec
-        d_o = dh * tc * o * (1.0 - o)
-        dc = dc_next + dh * o * (1.0 - tc * tc)
-        d_i = dc * gg * i * (1.0 - i)
-        d_f = dc * cs[s] * f * (1.0 - f)
-        d_g = dc * i * (1.0 - gg * gg)
-        dc_next = dc * f
-        d_gates[s] = np.concatenate((d_i, d_f, d_g, d_o), 1)
-        dh_rec = d_gates[s] @ whh
+    d_gates, dh_rec, dc_next = scan_backward(gates, cs, p["l2.weight_hh"], d_h_head)
     d_gin = d_gates.reshape(T, repeat, B, 4 * H).sum(1)
     if want_wgrad:
-        g["l2.weight_hh"] = np.einsum("sbg,sbh->gh", d_gates, hs[:-1])
-        g["l2.weight_ih"] = np.einsum("tbg,tbh->gh", d_gin, z1)
+        g["l2.weight_hh"] = wgrad(d_gates, hs[:-1])
+        g["l2.weight_ih"] = wgrad(d_gin, z1)
         g["l2.bias_ih"] = d_gin.sum((0, 1))
         g["l2.bias_hh"] = g["l2.bias_ih"].copy()
     d_p1 = (d_gin @ p["l2.weight_ih"]) * (1.0 - z1 * z1)
     if want_wgrad:
-        g["l1.weight"] = np.einsum("tbh,tbi->hi", d_p1, x)
+        g["l1.weight"] = wgrad(d_p1, x)
         g["l1.bias"] = d_p1.sum((0, 1))
     dx = d_p1 @ p["l1.weight"] if want_dx else None
     return g, dx, {"d_gates": d_gates, "d_h_head": d_h_head, "d_p1": d_p1, "dh0": dh_rec, "dc0": dc_next}

@@ -1693,18 +1693,27 @@ int lstm_scan_error_status(int* out, cudaStream_t stream) {
   return R2D2_OK;
 }
 
-int lstm_scan_max_active_clusters(int H, int nb, int backward) {
-  if (H == 256 && nb == 16) return backward ? max_active_clusters(lstm_scan_bwd_tc_kernel<256, 16>, 8, TcBwdSmem<256, 16>::BYTES)
-                                           : max_active_clusters(lstm_scan_fwd_tc_kernel<256, 16>, 8, TcFwdSmem<256, 16>::BYTES);
-  if (H == 256 && nb == 32) return backward ? max_active_clusters(lstm_scan_bwd_tc_kernel<256, 32>, 8, TcBwdSmem<256, 32>::BYTES)
-                                           : max_active_clusters(lstm_scan_fwd_tc_kernel<256, 32>, 8, TcFwdSmem<256, 32>::BYTES);
-  if (H == 512 && nb == 16) return backward ? max_active_clusters(lstm_scan_bwd_tc_kernel<512, 16>, 16, TcBwdSmem<512, 16>::BYTES)
-                                           : max_active_clusters(lstm_scan_fwd_tc_kernel<512, 16>, 16, TcFwdSmem<512, 16>::BYTES);
-  if (H == 512 && nb == 32) return backward ? max_active_clusters(lstm_scan_bwd_tc_kernel<512, 32>, 16, TcBwdSmem<512, 32>::BYTES)
-                                           : max_active_clusters(lstm_scan_fwd_tc_kernel<512, 32>, 16, TcFwdSmem<512, 32>::BYTES);
-  if (H == 128 && nb == 16) return backward ? max_active_clusters(lstm_scan_bwd_tc_kernel<128, 16>, 4, TcBwdSmem<128, 16>::BYTES)
-                                           : max_active_clusters(lstm_scan_fwd_tc_kernel<128, 16>, 4, TcFwdSmem<128, 16>::BYTES);
+// the same queries pick_tiling, bwd_tc and fwd_big make, so that tests can predict the tiling of a batch size
+template <int H>
+int max_active_clusters_tc(int nb, int backward) {
+  if (nb == 16) return backward ? max_active_clusters(lstm_scan_bwd_tc_kernel<H, 16>, H / 32, TcBwdSmem<H, 16>::BYTES)
+                                : max_active_clusters(lstm_scan_fwd_tc_kernel<H, 16>, H / 32, TcFwdSmem<H, 16>::BYTES);
+  if (nb == 32) return backward ? max_active_clusters(lstm_scan_bwd_tc_kernel<H, 32>, H / 32, TcBwdSmem<H, 32>::BYTES)
+                                : max_active_clusters(lstm_scan_fwd_tc_kernel<H, 32>, H / 32, TcFwdSmem<H, 32>::BYTES);
   return -1;
+}
+
+int lstm_scan_max_active_clusters(int H, int nb, int backward) {
+  if (H == 512 && nb == 80 && !backward)
+    return max_active_clusters(lstm_scan_fwd_big_kernel<false>, 16, BigFwdSmem::BYTES, BIG_THREADS);
+  switch (H) {
+    case 32: return max_active_clusters_tc<32>(nb, backward);
+    case 64: return max_active_clusters_tc<64>(nb, backward);
+    case 128: return max_active_clusters_tc<128>(nb, backward);
+    case 256: return max_active_clusters_tc<256>(nb, backward);
+    case 512: return max_active_clusters_tc<512>(nb, backward);
+    default: return -1;
+  }
 }
 
 int lstm_scan_forward_tc(const ScanFwdParams& p, cudaStream_t stream) {
