@@ -291,6 +291,28 @@ int r2d2_learner_set_step_count(r2d2_learner_t* l, int step);
 /* number of kernels launched by the three phases of one iteration (bench.py's gpu_launches) */
 int r2d2_learner_launches_per_iteration(r2d2_learner_t* l);
 
+/* ------------------------------------------------------------------------------------------------
+ * Batched acting (the per-step loop body of actor.py:136-148 over B environments): one step of actor, target actor,
+ * critic and target critic.  The critics are fed the UN-noised actions of their actors; noise and clipping stay on
+ * the host (actor.py:146-148).  Supported: H a multiple of 32 in [32, 512], O >= 1, 1 <= A <= 32,
+ * 1 <= B <= max_batch; anything else is rejected before any CUDA call.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct r2d2_act r2d2_act_t;
+
+/* shape: obs_size, n_actions, hidden (is_critic ignored) */
+int r2d2_act_create(r2d2_act_t** out, const r2d2_net_shape* shape, int max_batch);
+int r2d2_act_destroy(r2d2_act_t* a);
+/* flat DEVICE parameter blocks (state_dict order, see above) of actor, target_actor, critic, target_critic -> the
+ * handle's packed weight images.  Stream-ordered; the blocks may be freed once the stream has passed this call. */
+int r2d2_act_load(r2d2_act_t* a, const float* actor, const float* target_actor, const float* critic,
+                  const float* target_critic, r2d2_stream_t stream);
+/* obs [B,O]; state_in / state_out [4,2,B,H] in replay order (actor, target_actor, critic, target_critic) x (h, c),
+ * 16-byte aligned; state_out must not alias state_in; mu [B,A] = the actor's un-noised action.  4 launches. */
+int r2d2_act_step(r2d2_act_t* a, const float* obs, const float* state_in, float* state_out, float* mu, int B,
+                  r2d2_stream_t stream);
+/* *status != 0 if a bounded mbarrier wait inside an act kernel ever timed out; synchronises the stream */
+int r2d2_act_status(r2d2_act_t* a, int* status, r2d2_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -5,6 +5,9 @@ The actor is OUTSIDE the accelerated hot path (SURVEY 8: CPU actors stay as they
 exists so the reference's r2d2.py imports and runs unchanged, and it keeps the episode tuple, recurrent
 state and memory{i}.pt formats the learner ingests.  Without dm_control it steps a synthetic
 environment of the configured shape (BASELINE.json configs[4]: "Humanoid-shape synthetic env").
+
+With R2D2_ACTOR_ENVS=n, actor_process runs VecActor instead: n environments in lockstep, the four nets stepped on a
+GPU in one batched call per vector step (r2d2_b200.acting.ActEngine).  Unset, it is the CPU Actor below.
 """
 import os
 from collections import deque
@@ -61,7 +64,8 @@ def _make_env(actor_id):
 
 
 def actor_process(actor_id):
-    actor = Actor(actor_id)
+    n_envs = os.environ.get("R2D2_ACTOR_ENVS")
+    actor = VecActor(actor_id, int(n_envs)) if n_envs else Actor(actor_id)
     actor.run()
 
 
@@ -177,3 +181,126 @@ class Actor:
                 self.memory.add(self.sequence, self.recurrent_state, self.priority)
             if len(self.memory.memory) > self.memory_save_interval:
                 self.memory.save(self.actor_id)
+
+
+class VecActor:
+    """`n_envs` environments stepped in lockstep with the four nets on the GPU (r2d2_b200.acting.ActEngine: one
+    batched step per vector step instead of four batch-1 calls per environment).  Selected by actor_process when
+    R2D2_ACTOR_ENVS is set; writes the same episode tuples, recurrent states and memory{i}.pt files as Actor.
+
+    Env k gets seed actor_id * n_envs + k, and the exploration noise is one np.random.normal(0, 0.3, (n_envs, A)) draw
+    per vector step, so n_envs = 1 reproduces Actor's seeds and noise sequence.  Episodes that finish in the same step
+    get their n-step rewards and initial priorities from ONE batched r2d2_b200.actor_priority.episode_priorities call.
+    Device: R2D2_ACTOR_DEVICE if it names a CUDA device, else cuda:0."""
+
+    def __init__(self, actor_id, n_envs):
+        from r2d2_b200.acting import ActEngine
+        if n_envs < 1:
+            raise ValueError("n_envs >= 1")
+        self.actor_id, self.n_envs = actor_id, n_envs
+        self.envs = [_make_env(actor_id * n_envs + k) for k in range(n_envs)]
+        self.action_size = self.envs[0].action_spec().shape[0]
+        self.obs_size = get_obs(self.envs[0].reset().observation).shape[1]
+        self.burn_in_length, self.learning_length, self.n_step = 20, 40, 5
+        self.sequence_length = self.burn_in_length + self.learning_length
+        self.memory_sequence_size = 1000
+        self.memory = ReplayMemory(memory_sequence_size=self.memory_sequence_size)
+        self.memory_save_interval = 3
+        self.gamma = 0.997
+        self.actor_parameter_update_interval = 500
+        self.model_path = './model_data/'
+        self.hidden = int(os.environ.get("R2D2_HIDDEN", 128))
+        dev = os.environ.get("R2D2_ACTOR_DEVICE", "")
+        self.device = torch.device(dev if dev.startswith("cuda") else "cuda:0")
+        # the same freshly initialised nets as Actor (same torch RNG draws) until model.pt exists
+        actor = ActorNet(self.obs_size, self.action_size, 0, hidden=self.hidden)
+        critic = CriticNet(self.obs_size, self.action_size, 0, hidden=self.hidden)
+        self.weights = {"actor": actor.state_dict(), "target_actor": deepcopy(actor.state_dict()),
+                        "critic": critic.state_dict(), "target_critic": deepcopy(critic.state_dict())}
+        self.engine = ActEngine(self.obs_size, self.action_size, self.hidden, n_envs, self.device)
+        self.engine.load(self.weights)
+        self.load_model()
+
+    def load_model(self):
+        """Follow the learner's model.pt (actor.py:50-72); retried while the file is being replaced."""
+        path = self.model_path + 'model.pt'
+        if not os.path.isfile(path):
+            return
+        for _ in range(20):
+            try:
+                model_dict = torch.load(path, map_location="cpu")
+                weights = {name: model_dict[name] for name in ("actor", "target_actor", "critic", "target_critic")}
+                break
+            except Exception:
+                sleep(np.random.rand() * 2 + 0.5)
+        else:
+            return
+        self.weights = weights
+        self.engine.load(weights)
+
+    def _finish(self, done, seqs, states):
+        """Pad, n-step rewards and priorities of the episodes of envs `done` (one batched call), memory.add, save."""
+        from r2d2_b200 import actor_priority
+        keep = [k for k in done if len(seqs[k]) >= self.sequence_length]
+        if keep:
+            for k in keep:                                                    # actor.py:173
+                seqs[k].extend([(np.zeros(self.obs_size, np.float32), np.zeros(self.action_size, np.float32), [0.0], [1.0])
+                                for _ in range(self.n_step)])
+            episodes = [(np.stack([r[0] for r in seqs[k]]), np.stack([r[1] for r in seqs[k]]),
+                         np.asarray([r[2][0] for r in seqs[k]], np.float32),
+                         np.asarray([r[3][0] for r in seqs[k]], np.float32)) for k in keep]
+            prios, rews = actor_priority.episode_priorities(
+                self.weights["critic"], self.weights["target_actor"], self.weights["target_critic"], episodes,
+                hidden=self.hidden, burn_in=self.burn_in_length, learning=self.learning_length, n_step=self.n_step,
+                gamma=self.gamma, rewards_are_raw=True, device=self.device)
+            for k, pr, rw in zip(keep, prios, rews):
+                for i, row in enumerate(seqs[k]):
+                    row[2][0] = float(rw[i])
+                self.memory.add(seqs[k], states[k], [float(p) for p in pr])
+        if len(self.memory.memory) > self.memory_save_interval:
+            self.memory.save(self.actor_id)
+
+    def run(self, max_episodes=None):
+        """Step until `max_episodes` episodes (over all envs) have finished; forever for None."""
+        n, A = self.n_envs, self.action_size
+        obs = np.stack([get_obs(env.reset().observation)[0] for env in self.envs]).astype(np.float32)
+        self.engine.reset()
+        seqs, states = [[] for _ in range(n)], [[] for _ in range(n)]
+        reward_sum = np.zeros(n)
+        episode = step = 0
+        while max_episodes is None or episode < max_episodes:
+            mu, pre = self.engine.step(obs)                                   # pre-step states [4,2,n,H]
+            action = np.clip(mu + np.random.normal(0, 0.3, (n, A)), -1, 1)
+            nxt = obs.copy()
+            done = []
+            for k, env in enumerate(self.envs):
+                reward = 0.0
+                for _ in range(4):                                            # action repeat, actor.py:152-157
+                    time_step = env.step(action[k])
+                    reward += time_step.reward or 0.0
+                    if time_step.last():
+                        break
+                nxt[k] = get_obs(time_step.observation)[0]
+                last = time_step.last()
+                reward_sum[k] += reward
+                seqs[k].append((obs[k].copy(), action[k].astype(np.float32), [reward], [1.0 if last else 0.0]))
+                st = pre[:, :, k].copy()
+                states[k].append([[st[i, 0], st[i, 1]] for i in range(4)])
+                if last:
+                    done.append(k)
+            step += 1
+            if step % self.actor_parameter_update_interval == 0:
+                self.load_model()
+            if done:
+                episode += len(done)
+                if self.actor_id == 0:
+                    print('episodes:', episode, 'step:', step, 'reward:', float(np.mean(reward_sum[done])))
+                self._finish(done, seqs, states)
+                mask = np.zeros(n, bool)
+                for k in done:
+                    nxt[k] = get_obs(self.envs[k].reset().observation)[0]
+                    seqs[k], states[k] = [], []
+                    reward_sum[k] = 0.0
+                    mask[k] = True
+                self.engine.reset(mask)
+            obs = nxt

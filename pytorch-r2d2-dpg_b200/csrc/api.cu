@@ -1,6 +1,7 @@
 // extern "C" surface of libr2d2_b200 (declared in include/r2d2_b200.h).
 #include <atomic>
 
+#include "act.cuh"
 #include "common.cuh"
 #include "elementwise.cuh"
 #include "gemm.cuh"
@@ -309,6 +310,25 @@ int r2d2_learner_launches_per_iteration(r2d2_learner_t* lh) {
   Learner* l = reinterpret_cast<Learner*>(lh);
   return l->launches_phase[0] + l->launches_phase[1] + l->launches_phase[2] +
          (l->target_phase_standalone ? l->launches_target : 0);
+}
+
+// ---- batched acting ----
+int r2d2_act_create(r2d2_act_t** out, const r2d2_net_shape* shape, int max_batch) {
+  R2D2_REQUIRE(out && shape, "null");
+  return act_create(reinterpret_cast<Act**>(out), shape->obs_size, shape->n_actions, shape->hidden, max_batch);
+}
+int r2d2_act_destroy(r2d2_act_t* a) { return act_destroy(reinterpret_cast<Act*>(a)); }
+int r2d2_act_load(r2d2_act_t* a, const float* actor, const float* target_actor, const float* critic,
+                  const float* target_critic, r2d2_stream_t stream) {
+  const float* const params[4] = {actor, target_actor, critic, target_critic};
+  return act_load(reinterpret_cast<Act*>(a), params, S(stream));
+}
+int r2d2_act_step(r2d2_act_t* a, const float* obs, const float* state_in, float* state_out, float* mu, int B,
+                  r2d2_stream_t stream) {
+  return act_step(reinterpret_cast<Act*>(a), obs, state_in, state_out, mu, B, S(stream));
+}
+int r2d2_act_status(r2d2_act_t* a, int* status, r2d2_stream_t stream) {
+  return act_status(reinterpret_cast<Act*>(a), status, S(stream));
 }
 
 }  // extern "C"

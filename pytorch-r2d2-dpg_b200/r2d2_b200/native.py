@@ -130,6 +130,11 @@ SIGNATURES = {
     "r2d2_learner_peer_counters": (c_int, [c_void_p, c_void_p, c_int, c_void_p]),
     "r2d2_learner_peer_status": (c_int, [c_void_p, POINTER(c_int), c_void_p]),
     "r2d2_learner_launches_per_iteration": (c_int, [c_void_p]),
+    "r2d2_act_create": (c_int, [POINTER(c_void_p), POINTER(NetShape), c_int]),
+    "r2d2_act_destroy": (c_int, [c_void_p]),
+    "r2d2_act_load": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "r2d2_act_step": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
+    "r2d2_act_status": (c_int, [c_void_p, POINTER(c_int), c_void_p]),
 }
 
 _lib = None
